@@ -4,6 +4,7 @@ ColBERT max-sim, dim=128, Lq=32, Ld=180, 64 queries x 1000 docs per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload colbert|tk|knrm|tkl|bert_dot]     (default colbert = the BASELINE metric)
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL).  Prints ONE JSON line on rank 0.
 
@@ -181,6 +182,9 @@ class ColbertWorkload:
         from matchmaker_b200 import interaction
         return interaction.maxsim(self.cq, self.cd, self.cqm, self.cdm, docs_per_query=DOCS_PER_QUERY, impl="tcgen05")
 
+    def outputs(self, out):
+        return {"scores": out}
+
     def exchange(self, s):
         from matchmaker_b200 import sharding
         return sharding.topk_all_gather_merge(s.view(N_QUERIES, DOCS_PER_QUERY), TOPK, self.id_base)
@@ -293,6 +297,9 @@ class KernelPoolWorkload:
         from matchmaker_b200 import interaction
         return interaction.kernel_pool(*self.c, alpha=self.calpha, log_scale=self.log_scale)["score"]
 
+    def outputs(self, out):
+        return {"scores": out}
+
     def exchange(self, s):
         return s  # re-ranking pairs are independent: no data-path collective
 
@@ -362,7 +369,12 @@ class KernelPoolTrainWorkload(KernelPoolWorkload):
         score, _ = autograd.kernel_pool(self.c[0], self.c[1], self.c[2], self.c[3], self.c[4], self.c[5], self.c[6], self.calpha,
                                         self.log_scale)
         score.backward(self.gout)
+        self.score = score.detach()   # detached: a kept autograd graph would break the CUDA-graph capture of the next step
         return self.c[0].grad
+
+    def outputs(self, out):
+        return {"scores": self.score, "grad_q": self.c[0].grad, "grad_d": self.c[1].grad, "grad_weight": self.c[6].grad,
+                "grad_alpha": self.calpha.grad}
 
     def e2e_step(self):
         from matchmaker_b200 import autograd
@@ -449,6 +461,9 @@ class TklWorkload:
         c = self.c
         return self._run(c["q"], c["qm"], c["ch"], c["cm"], c["pk"])
 
+    def outputs(self, out):
+        return {"scores": out}
+
     def exchange(self, s):
         return s
 
@@ -506,6 +521,9 @@ class BertDotWorkload:
     def kernel_step(self):
         from matchmaker_b200 import interaction
         return interaction.flat_ip_topk(self.cq, self.cp, self.k, id_base=self.id_base)
+
+    def outputs(self, out):
+        return {"scores": out[0], "ids": out[1]}
 
     def exchange(self, si):
         from matchmaker_b200 import sharding
@@ -783,6 +801,28 @@ def bench_secondary(name, dev, steps, cpu_budget_s):
     return rec
 
 
+DUMP_SAMPLE = 1 << 22          # elements kept of a larger output (16 MB in float32)
+DUMP_LIMIT = 64 << 20          # bytes written by --dump-outputs in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each output of the last timed step as out_dir/<name>.npy: floating-point outputs as float32, integer ones
+    (ids) as float64, which holds them exactly.  An output of more than DUMP_SAMPLE elements is written as the same
+    seeded sample of its flattened elements on every run, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(SEED))[:DUMP_SAMPLE].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64)
+        total += a.nbytes
+        assert total <= DUMP_LIMIT, "--dump-outputs: more than %d bytes" % DUMP_LIMIT
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -795,7 +835,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="never replay the step from a CUDA graph")
     ap.add_argument("--no-secondary", action="store_true",
                     help="skip the per-workload sub-records (tk, knrm, tkl, bert_dot, ...) of the default N=1 run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what rank 0's last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -880,6 +926,8 @@ def main():
     e1.record()
     sync_all()
     t_val1 = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl.outputs(out))
     ms_total = e0.elapsed_time(e1)
     kern_ms = statistics.mean(a.elapsed_time(b) for a, b in kern_ev)
     t = torch.tensor([ms_total, kern_ms], device=dev, dtype=torch.float64)

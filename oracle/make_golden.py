@@ -269,13 +269,34 @@ def golden_conv_knrm():
           **{f"qg{i}": t for i, t in enumerate(qg)}, **{f"dg{i}": t for i, t in enumerate(dg)}, **state)
 
 
+def golden_regen():
+    """A second run of the reference's classes on the inputs of two committed fixtures (knrm_small, colbert_small):
+    tests/test_oracle_golden.py checks the fixtures against it without needing the reference sources."""
+    def load(name):
+        z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
+        return {k: torch.from_numpy(z[k]) for k in z.files}
+
+    g = load("knrm_small")
+    ref = R.load_knrm(11)
+    with torch.no_grad():
+        ref.dense.weight.copy_(g["weight"].view(1, -1))
+        knrm = ref.forward(g["q"], g["d"], g["q_mask"], g["d_mask"])
+    _, inst = R.load_colbert()
+    c = load("colbert_small")
+    with torch.no_grad():
+        colbert = inst.forward({"vecs": c["q"].clone(), "attention_mask": c["q_mask"]},
+                               {"vecs": c["d"].clone(), "attention_mask": c["d_mask"]}, use_fp16=False)
+    _save("reference_regen", knrm_small_score=knrm, colbert_small_score=colbert)
+
+
 def main():
     if not R.reference_available():
         print("reference not mounted at", R.REFERENCE_ROOT, "- cannot regenerate golden vectors", file=sys.stderr)
         return 1
     only = set(sys.argv[1:])   # e.g. `python -m oracle.make_golden knrm` regenerates one family
     for name, fn in (("knrm", golden_knrm), ("tk", golden_tk), ("tkl", golden_tkl), ("colbert", golden_colbert),
-                     ("bert_dot", golden_bert_dot), ("tk_sparse", golden_tk_sparse), ("conv_knrm", golden_conv_knrm)):
+                     ("bert_dot", golden_bert_dot), ("tk_sparse", golden_tk_sparse), ("conv_knrm", golden_conv_knrm),
+                     ("regen", golden_regen)):
         if not only or name in only:
             fn()
     return 0
