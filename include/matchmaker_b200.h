@@ -89,8 +89,10 @@ MMB200_API int mmb200_device_info(int device, int* sm_count, int* cc_major, int*
  * pair_dmask [n_pairs] int32 or NULL: row of d_mask applied to pair p (default di).  Exists only
  *        to reproduce colbert.py:158, which indexes the document mask by the QUERY position.
  * out    [n_pairs] float32
- * argmax [n_pairs, Lq] int32 or NULL: index j* of the max per query token (-1 when the query
- *        token is masked or every document position is masked) -- what backward needs.
+ * argmax [n_pairs, Lq] int32 or NULL: index j* of the first max per query token (-1 when the
+ *        query token is masked or the -1000 fill is the max) -- what backward needs.
+ * Envelope: 1 <= Lq <= 128, 1 <= dim <= 1024, Ld >= 1 (else MMB200_ERR_INVALID); IMPL_AUTO serves
+ *        all of it, a forced impl returns MMB200_ERR_UNSUPPORTED where its kernel does not apply.
  * ------------------------------------------------------------------------------------------ */
 MMB200_API int mmb200_maxsim_fwd(const void* q, const void* d, const void* q_mask, const void* d_mask,
                       const int32_t* pair_q, const int32_t* pair_d, const int32_t* pair_dmask,

@@ -24,8 +24,12 @@
 //     running max over the tiles of a pair in registers, cross-warp combine through 2 KB of
 //     shared memory, query mask, warp-sum, one fp32 store per pair.
 //
-// Kernel `maxsim_simt_kernel`: CUDA-core version for any dtype / dim / length (fp32 inputs,
-// dim % 64 != 0, argmax for backward); also the in-library cross-check of the tensor-core path.
+// Kernel `maxsim_simt_kernel`: CUDA-core version for every shape of the envelope (fp32 inputs,
+// dim % 64 != 0, argmax for backward, query tiles too large for the tensor-core kernels); also the
+// in-library cross-check of the tensor-core path.
+//
+// Envelope of mmb200_maxsim_fwd: 1 <= Lq <= 128, 1 <= dim <= 1024, any Ld >= 1; shapes outside it
+// are rejected up front.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -65,58 +69,66 @@ constexpr float kMaskedScore = -1000.0f;  // colbert.py:69
 
 // ---------------------------------------------------------------------------------------------
 // SIMT kernel: one CTA (128 threads) per pair.  Q is staged in shared memory as fp32 with a
-// padded row stride; warp w takes document rows w, w+4, ...; lane l owns query tokens l, l+32, ...
+// padded row stride, `qrows` query rows per pass (all Lq rows when they fit, else a multiple of
+// 32); per pass warp w takes document rows w, w+4, ...; lane l owns the pass's query rows l, l+32,
+// ...  Each (query row, document row) dot product is the same fmaf chain over k whatever the pass
+// size, so scores and argmax do not depend on how many passes a shape needs.
 // ---------------------------------------------------------------------------------------------
 constexpr int kSimtThreads = 128;
 constexpr int kSimtMaxQPerLane = 4;  // Lq <= 128
+constexpr int kMaxsimMaxLq = 32 * kSimtMaxQPerLane;
+constexpr int kMaxsimMaxDim = 1024;
 
 template <typename T>
-__global__ void __launch_bounds__(kSimtThreads) maxsim_simt_kernel(MaxsimParams P) {
+__global__ void __launch_bounds__(kSimtThreads) maxsim_simt_kernel(MaxsimParams P, int qrows) {
   extern __shared__ float smem_f[];
   const int Lq = P.Lq, Ld = P.Ld, dim = P.dim;
   const int qstride = dim + 1;
-  float* sq = smem_f;                          // [Lq][dim+1]
-  float* smax = sq + (size_t)Lq * qstride;     // [4][Lq]
+  float* sq = smem_f;                          // [qrows][dim+1]
+  float* smax = sq + (size_t)qrows * qstride;  // [4][Lq]
   int* sarg = reinterpret_cast<int*>(smax + 4 * Lq);  // [4][Lq]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   for (int64_t p = blockIdx.x; p < P.n_pairs; p += gridDim.x) {
     const int64_t qi = pair_query(P, p), di = pair_doc(P, p), dmi = pair_dmask_row(P, p);
-    const T* qptr = static_cast<const T*>(P.q) + qi * (int64_t)Lq * dim;
     const T* dptr = static_cast<const T*>(P.d) + di * (int64_t)Ld * dim;
-    __syncthreads();
-    for (int e = threadIdx.x; e < Lq * dim; e += kSimtThreads) {
-      sq[(e / dim) * qstride + (e % dim)] = to_float(qptr[e]);
-    }
-    __syncthreads();
-    float best[kSimtMaxQPerLane];
-    int barg[kSimtMaxQPerLane];
+    for (int r0 = 0; r0 < Lq; r0 += qrows) {
+      const int nr = min(qrows, Lq - r0);
+      const T* qptr = static_cast<const T*>(P.q) + (qi * (int64_t)Lq + r0) * dim;
+      __syncthreads();
+      for (int e = threadIdx.x; e < nr * dim; e += kSimtThreads) {
+        sq[(e / dim) * qstride + (e % dim)] = to_float(qptr[e]);
+      }
+      __syncthreads();
+      float best[kSimtMaxQPerLane];
+      int barg[kSimtMaxQPerLane];
 #pragma unroll
-    for (int t = 0; t < kSimtMaxQPerLane; ++t) { best[t] = -INFINITY; barg[t] = -1; }
-    for (int j = warp; j < Ld; j += 4) {
-      const bool ok = mask_at(P.d_mask, P.d_mask ? P.mask_dtype : MMB200_MASK_NONE, dmi * (int64_t)Ld + j);
-      float acc[kSimtMaxQPerLane] = {0.f, 0.f, 0.f, 0.f};
-      if (ok) {
-        const T* drow = dptr + (int64_t)j * dim;
-        for (int k = 0; k < dim; ++k) {
-          const float dv = to_float(drow[k]);
+      for (int t = 0; t < kSimtMaxQPerLane; ++t) { best[t] = -INFINITY; barg[t] = -1; }
+      for (int j = warp; j < Ld; j += 4) {
+        const bool ok = mask_at(P.d_mask, P.d_mask ? P.mask_dtype : MMB200_MASK_NONE, dmi * (int64_t)Ld + j);
+        float acc[kSimtMaxQPerLane] = {0.f, 0.f, 0.f, 0.f};
+        if (ok) {
+          const T* drow = dptr + (int64_t)j * dim;
+          for (int k = 0; k < dim; ++k) {
+            const float dv = to_float(drow[k]);
 #pragma unroll
-          for (int t = 0; t < kSimtMaxQPerLane; ++t) {
-            const int i = lane + 32 * t;
-            if (i < Lq) acc[t] = fmaf(sq[i * qstride + k], dv, acc[t]);
+            for (int t = 0; t < kSimtMaxQPerLane; ++t) {
+              const int i = lane + 32 * t;
+              if (i < nr) acc[t] = fmaf(sq[i * qstride + k], dv, acc[t]);
+            }
           }
+        }
+#pragma unroll
+        for (int t = 0; t < kSimtMaxQPerLane; ++t) {
+          const float v = ok ? acc[t] : kMaskedScore;
+          if (v > best[t]) { best[t] = v; barg[t] = ok ? j : -1; }
         }
       }
 #pragma unroll
       for (int t = 0; t < kSimtMaxQPerLane; ++t) {
-        const float v = ok ? acc[t] : kMaskedScore;
-        if (v > best[t]) { best[t] = v; barg[t] = ok ? j : -1; }
+        const int i = lane + 32 * t;
+        if (i < nr) { smax[warp * Lq + r0 + i] = best[t]; sarg[warp * Lq + r0 + i] = barg[t]; }
       }
-    }
-#pragma unroll
-    for (int t = 0; t < kSimtMaxQPerLane; ++t) {
-      const int i = lane + 32 * t;
-      if (i < Lq) { smax[warp * Lq + i] = best[t]; sarg[warp * Lq + i] = barg[t]; }
     }
     __syncthreads();
     if (warp == 0) {
@@ -429,17 +441,9 @@ maxsim_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-static bool tc_supported(const MaxsimParams& P, int dtype, std::string* why) {
-  if (dtype != MMB200_F16 && dtype != MMB200_BF16) { *why = "tcgen05 path needs f16/bf16 inputs"; return false; }
-  if (P.dim % 64 != 0 || P.dim < 64 || P.dim > 1024) { *why = "tcgen05 path needs dim % 64 == 0, 64 <= dim <= 1024"; return false; }
-  if (P.Lq < 1 || P.Lq > 128) { *why = "tcgen05 path needs 1 <= Lq <= 128"; return false; }
-  if (P.Ld < 1) { *why = "Ld < 1"; return false; }
-  if (P.argmax) { *why = "argmax output is produced by the SIMT kernel"; return false; }
-  if ((reinterpret_cast<uintptr_t>(P.q) | reinterpret_cast<uintptr_t>(P.d)) & 15) { *why = "q/d must be 16-byte aligned"; return false; }
-  return true;
-}
-
-static int launch_tc(const MaxsimParams& P, int dtype, const DeviceInfo& dev, cudaStream_t stream) {
+// Launch geometry of maxsim_tc_kernel; L.stages < 2 means the two query slots leave no room for a
+// double-buffered document ring in shared memory.
+static TcLaunch tc_plan(const MaxsimParams& P, int dtype, const DeviceInfo& dev, size_t* smem_bytes) {
   TcLaunch L;
   L.npad = ((P.Lq + 31) / 32) * 32;
   L.kblocks = P.dim / 64;
@@ -453,12 +457,30 @@ static int launch_tc(const MaxsimParams& P, int dtype, const DeviceInfo& dev, cu
   const int stage_bytes = L.kbs * kKBlockBytes;
   const int fixed = kQSlots * L.qslot_bytes + (int)sizeof(TcShared) + 1024 /* alignment slack */;
   const int budget = dev.max_smem_optin - fixed;
-  L.stages = std::min(kMaxStages, budget / stage_bytes);
-  if (L.stages < 2) {
-    set_error("maxsim tcgen05: query tile too large for shared memory");
-    return MMB200_ERR_UNSUPPORTED;
+  L.stages = budget < 0 ? 0 : std::min(kMaxStages, budget / stage_bytes);
+  *smem_bytes = (size_t)L.stages * stage_bytes + fixed;
+  return L;
+}
+
+static bool tc_supported(const MaxsimParams& P, int dtype, const DeviceInfo& dev, std::string* why) {
+  if (dtype != MMB200_F16 && dtype != MMB200_BF16) { *why = "tcgen05 path needs f16/bf16 inputs"; return false; }
+  if (P.dim % 64 != 0 || P.dim < 64 || P.dim > 1024) { *why = "tcgen05 path needs dim % 64 == 0, 64 <= dim <= 1024"; return false; }
+  if (P.Lq < 1 || P.Lq > 128) { *why = "tcgen05 path needs 1 <= Lq <= 128"; return false; }
+  if (P.Ld < 1) { *why = "Ld < 1"; return false; }
+  if (P.argmax) { *why = "argmax output is produced by the SIMT kernel"; return false; }
+  if ((reinterpret_cast<uintptr_t>(P.q) | reinterpret_cast<uintptr_t>(P.d)) & 15) { *why = "q/d must be 16-byte aligned"; return false; }
+  size_t smem_bytes;
+  if (tc_plan(P, dtype, dev, &smem_bytes).stages < 2) {
+    *why = "tcgen05 path: the query tile (2 x dim/64 x round32(Lq) x 128 B) leaves no room for two document stages in shared memory";
+    return false;
   }
-  const size_t smem_bytes = (size_t)L.stages * stage_bytes + fixed;
+  return true;
+}
+
+// Only called for shapes that tc_supported() accepts.
+static int launch_tc(const MaxsimParams& P, int dtype, const DeviceInfo& dev, cudaStream_t stream) {
+  size_t smem_bytes;
+  const TcLaunch L = tc_plan(P, dtype, dev, &smem_bytes);
 
   const CUtensorMapDataType tdt = dtype == MMB200_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
   CUtensorMap tq, td;
@@ -491,15 +513,19 @@ static int launch_tc(const MaxsimParams& P, int dtype, const DeviceInfo& dev, cu
 }
 
 static int launch_simt(const MaxsimParams& P, int dtype, const DeviceInfo& dev, cudaStream_t stream) {
-  MMB_REQUIRE(P.Lq <= 32 * kSimtMaxQPerLane, "SIMT max-sim kernel supports Lq <= 128");
-  const size_t smem_bytes = ((size_t)P.Lq * (P.dim + 1) + 8 * (size_t)P.Lq) * sizeof(float);
-  MMB_REQUIRE(smem_bytes <= (size_t)dev.max_smem_optin, "query tile does not fit in shared memory");
+  // shared memory: qrows staged query rows of dim+1 floats + the per-warp [4][Lq] max and argmax
+  const size_t row_bytes = (size_t)(P.dim + 1) * sizeof(float), fixed = 8 * (size_t)P.Lq * sizeof(float);
+  int qrows = P.Lq;
+  if (fixed + (size_t)qrows * row_bytes > (size_t)dev.max_smem_optin)
+    qrows = (int)(((size_t)dev.max_smem_optin - fixed) / row_bytes) / 32 * 32;
+  MMB_REQUIRE(qrows >= 1, "SIMT max-sim: 32 query rows of this dim do not fit in shared memory");
+  const size_t smem_bytes = fixed + (size_t)qrows * row_bytes;
   const int grid = (int)std::min<int64_t>((int64_t)dev.sm_count * 8, P.n_pairs);
 #define MMB_LAUNCH_SIMT(T)                                                                                  \
   do {                                                                                                      \
     MMB_CHECK_CUDA(cudaFuncSetAttribute(maxsim_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                         (int)smem_bytes));                                                  \
-    maxsim_simt_kernel<T><<<grid, kSimtThreads, smem_bytes, stream>>>(P);                                  \
+    maxsim_simt_kernel<T><<<grid, kSimtThreads, smem_bytes, stream>>>(P, qrows);                           \
   } while (0)
   if (dtype == MMB200_F16) MMB_LAUNCH_SIMT(__half);
   else if (dtype == MMB200_BF16) MMB_LAUNCH_SIMT(__nv_bfloat16);
@@ -514,6 +540,7 @@ int maxsim_fwd_device(const MaxsimParams& P, int dtype, int impl, cudaStream_t s
   MMB_REQUIRE(dtype_size(dtype) != 0, "unknown dtype");
   MMB_REQUIRE(P.n_pairs >= 0 && P.n_q > 0 && P.n_d > 0, "bad counts");
   MMB_REQUIRE(P.Lq > 0 && P.Ld > 0 && P.dim > 0, "bad shape");
+  MMB_REQUIRE(P.Lq <= kMaxsimMaxLq && P.dim <= kMaxsimMaxDim, "max-sim supports 1 <= Lq <= 128 and 1 <= dim <= 1024");
   MMB_REQUIRE(P.docs_per_query >= 1, "docs_per_query must be >= 1");
   if ((P.q_mask || P.d_mask)) MMB_REQUIRE(mask_dtype_size(P.mask_dtype) != 0, "unknown mask dtype");
   if (!P.pair_q) MMB_REQUIRE((P.pair_base + P.n_pairs + P.docs_per_query - 1) / P.docs_per_query <= P.n_q, "n_pairs / docs_per_query exceeds n_q");
@@ -548,7 +575,7 @@ int maxsim_fwd_device(const MaxsimParams& P, int dtype, int impl, cudaStream_t s
     if (handled || rc != MMB200_OK) return rc;
   }
   std::string why;
-  const bool tc_ok = tc_supported(P, dtype, &why);
+  const bool tc_ok = tc_supported(P, dtype, dev, &why);
   if ((impl == MMB200_IMPL_TCGEN05 || impl == MMB200_IMPL_TCGEN05_DOCM) && !tc_ok) {
     set_error(why);
     return MMB200_ERR_UNSUPPORTED;

@@ -70,6 +70,13 @@ def maxsim(q: torch.Tensor, d: torch.Tensor, q_mask: Optional[torch.Tensor] = No
     q [n_q, Lq, dim], d [n_d, Ld, dim] (fp16 / bf16 / fp32, same dtype), masks [n, L] (nonzero =
     token).  Pair p scores query ``pair_q[p]`` (default ``p // docs_per_query``) against document
     ``pair_d[p]`` (default ``p``).  Semantics: matchmaker/models/colbert.py:68-75 / :100-112.
+
+    Envelope: 1 <= Lq <= 128, 1 <= dim <= 1024, any Ld >= 1, with or without ``return_argmax``; ``impl="auto"``
+    serves every such shape and raises :class:`MatchmakerB200Error` for any other.  ``impl="auto"`` picks the
+    queries-on-M tcgen05 kernel (fp16/bf16, Lq <= 32, dim 64 or 128, 16-byte aligned q/d), else the
+    documents-on-M tcgen05 kernel (fp16/bf16, dim % 64 == 0, no argmax, aligned, query tile small enough to
+    leave room for two document stages in shared memory: e.g. Lq <= 32 at dim 768), else the SIMT kernel.
+    A forced ``impl`` raises where its kernel does not cover the shape.
     """
     dev = _require_cuda(q, d, q_mask, d_mask, pair_q, pair_d, pair_dmask)
     if q.dtype != d.dtype or q.dtype not in _DTYPES:

@@ -221,7 +221,7 @@ def maxsim_allpairs_own_masks(q: torch.Tensor, q_mask: torch.Tensor, d: torch.Te
     [Nq,Nd,Lq,Ld] score tensor, so the reference masks pair (a,b) with the mask of document a
     (see maxsim_allpairs above, which keeps that quirk).  This is the intended semantics, built from
     the pair scorer colbert.py:68-75."""
-    out = torch.empty(q.shape[0], d.shape[0])
+    out = torch.empty(q.shape[0], d.shape[0], dtype=q.dtype)
     for a in range(q.shape[0]):
         n = d.shape[0]
         out[a] = maxsim_pairs(q[a:a + 1].expand(n, -1, -1), d, q_mask[a:a + 1].expand(n, -1), d_mask)

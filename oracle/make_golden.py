@@ -202,6 +202,21 @@ def golden_colbert():
     _save("colbert_cfg3", q=q, d=d, q_mask=qm, d_mask=dm, docs_per_query=np.array(3), score=score)
 
 
+def golden_colbert_768():
+    """The shape the reference's shipped ColBERT runs at: colbert_compression_dim 768, max_query_length 30,
+    max_doc_length 200 (config/train/models/colbert.yaml, config/train/defaults.yaml), fp16 storage upcast to fp32
+    like dense_retrieval.py:406; 2 queries x 2 docs."""
+    _, inst = R.load_colbert()
+    q, d, qm, dm = O.synth_colbert_inputs(2, 2, 30, 200, 768, seed=1768, dtype=torch.float16)
+    qe = q.float().repeat_interleave(2, dim=0)
+    qme = qm.repeat_interleave(2, dim=0)
+    with torch.no_grad():
+        score = inst.forward({"vecs": qe.clone(), "attention_mask": qme},
+                             {"vecs": d.float(), "attention_mask": dm}, use_fp16=False)
+    _check(O.maxsim_one_query_many_docs(q.float(), d.float(), qm, dm, 2), score, "colbert dim-768 shape")
+    _save("colbert_768", q=q, d=d, q_mask=qm, d_mask=dm, docs_per_query=np.array(2), score=score)
+
+
 def golden_bert_dot():
     cls, inst = R.load_bert_dot()
     inst.eval()
@@ -270,7 +285,7 @@ def golden_conv_knrm():
 
 
 def golden_regen():
-    """A second run of the reference's classes on the inputs of two committed fixtures (knrm_small, colbert_small):
+    """A second run of the reference's classes on the inputs of committed fixtures (knrm_small, colbert_small, colbert_768):
     tests/test_oracle_golden.py checks the fixtures against it without needing the reference sources."""
     def load(name):
         z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
@@ -286,7 +301,13 @@ def golden_regen():
     with torch.no_grad():
         colbert = inst.forward({"vecs": c["q"].clone(), "attention_mask": c["q_mask"]},
                                {"vecs": c["d"].clone(), "attention_mask": c["d_mask"]}, use_fp16=False)
-    _save("reference_regen", knrm_small_score=knrm, colbert_small_score=colbert)
+    c = load("colbert_768")
+    dpq = int(c["docs_per_query"])
+    with torch.no_grad():
+        colbert_768 = inst.forward({"vecs": c["q"].float().repeat_interleave(dpq, dim=0),
+                                    "attention_mask": c["q_mask"].repeat_interleave(dpq, dim=0)},
+                                   {"vecs": c["d"].float(), "attention_mask": c["d_mask"]}, use_fp16=False)
+    _save("reference_regen", knrm_small_score=knrm, colbert_small_score=colbert, colbert_768_score=colbert_768)
 
 
 def main():
@@ -294,7 +315,7 @@ def main():
         print("reference not mounted at", R.REFERENCE_ROOT, "- cannot regenerate golden vectors", file=sys.stderr)
         return 1
     only = set(sys.argv[1:])   # e.g. `python -m oracle.make_golden knrm` regenerates one family
-    for name, fn in (("knrm", golden_knrm), ("tk", golden_tk), ("tkl", golden_tkl), ("colbert", golden_colbert),
+    for name, fn in (("knrm", golden_knrm), ("tk", golden_tk), ("tkl", golden_tkl), ("colbert", golden_colbert), ("colbert_768", golden_colbert_768),
                      ("bert_dot", golden_bert_dot), ("tk_sparse", golden_tk_sparse), ("conv_knrm", golden_conv_knrm),
                      ("regen", golden_regen)):
         if not only or name in only:

@@ -63,6 +63,12 @@ def test_colbert_cfg3_shape():
     _eq(s, g["score"])
 
 
+def test_colbert_768_shape():
+    g = load_golden("colbert_768")
+    s = O.maxsim_one_query_many_docs(g["q"].float(), g["d"].float(), g["q_mask"], g["d_mask"], int(g["docs_per_query"]))
+    _eq(s, g["score"])
+
+
 def test_bert_dot():
     g = load_golden("bert_dot_small")
     _eq(O.dot_pairs(g["qv"], g["dv"]), g["score"])
@@ -95,6 +101,7 @@ def test_golden_regenerates_from_reference():
     r = load_golden("reference_regen")
     _eq(r["knrm_small_score"], load_golden("knrm_small")["score"])
     _eq(r["colbert_small_score"], load_golden("colbert_small")["score"])
+    _eq(r["colbert_768_score"], load_golden("colbert_768")["score"])
 
 
 def test_tk_sparse_interaction():
